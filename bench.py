@@ -20,17 +20,20 @@ times, work counters and the identity of the drop-in's SAM file with the referen
 from __future__ import annotations
 
 import argparse
+import atexit
 import json
 import os
 import re
 import shutil
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from
 
 import numpy as np
 
@@ -455,9 +458,10 @@ NSLOTS = int(os.environ.get("URMB_BENCH_SLOTS", "6"))   # batch slots the bench 
              # five steps to finish before its slot is needed again
 
 
-def time_steps(ctx, batches, paired, steps, warmup, D, device):
+def time_steps(ctx, batches, paired, steps, warmup, D, device, keep_last=False):
     """K steps issued back to back with the inputs resident in HBM: device time between two context-wide CUDA events,
-    per-kernel-class launch durations (CUDA events around every launch) of the last steps."""
+    per-kernel-class launch durations (CUDA events around every launch) of the last steps.  keep_last: also return
+    copies of the results of step K-1 (r1, r2, runs) as `last`."""
     import torch
     nb = len(batches)
     B = len(batches[0][4]) - 1
@@ -490,13 +494,47 @@ def time_steps(ctx, batches, paired, steps, warmup, D, device):
                 kms[name] = kms.get(name, 0.0) + v / nlast
                 klaunch[name] = klaunch.get(name, 0) + tm["kernel_launches"][name]
     klaunch = {k: max(1, v // nlast) for k, v in klaunch.items()}
-    for s in range(min(NSLOTS, steps)):   # drain (results are not looked at here)
+    last = None
+    for s in range(min(NSLOTS, steps)):   # drain
         ctx.download(s)
-        ctx.wait(s, B, paired)
+        r1, r2, runs = ctx.wait(s, B, paired)
+        if keep_last and s == (steps - 1) % NSLOTS:
+            last = (r1.copy(), None if r2 is None else r2.copy(), runs.copy())
     # pairs the probe kernel's first look finished (seed-loop exit of Search4/5) in the last batch of slot 0
     first_look = ctx.first_look_count(0)[0] / float(B) if paired else 0.0
     return {"dev_ms": dev_ms, "wall_ms": 1e3 * t_wall, "gpu_launches": gpu_launches, "kernel_ms": kms, "kernel_launches": klaunch,
-            "first_look_frac": first_look}
+            "first_look_frac": first_look, "last": last}
+
+
+DUMP_SAMPLE = 100_000   # reads per mate: 4 MB of result fields per mate, plus the path runs of those reads
+
+
+def dump_outputs(out_dir, last, seed=0):
+    """The results of one step as .npy files: for a fixed, seeded sample of the batch's reads (`sample_index`), every
+    result field per mate (`mate1_<field>`, `mate2_<field>` when paired; db_pos in float64, the rest in float32) and the
+    path runs of the sampled reads in sample order (`mateN_path`, `mateN_path_runs` long each).  The pool offsets of the
+    paths are left out: they depend on the order in which warps finish."""
+    r1, r2, runs = last
+    n = len(r1)
+    idx = np.sort(np.random.default_rng(seed).choice(n, size=min(n, DUMP_SAMPLE), replace=False))
+    arrays = {"sample_index": idx.astype(np.float64)}
+    for m, r in ((1, r1), (2, r2)):
+        if r is None:
+            continue
+        s = r[idx]
+        for f in ("db_pos", "score", "best", "second", "mapq", "flags", "hit_count", "hsp_count", "path_runs"):
+            arrays[f"mate{m}_{f}"] = s[f].astype(np.float64 if f == "db_pos" else np.float32)
+        lens = s["path_runs"].astype(np.int64)
+        starts = np.repeat(s["path_off"].astype(np.int64), lens)
+        within = np.arange(int(lens.sum())) - np.repeat(np.cumsum(lens) - lens, lens)
+        arrays[f"mate{m}_path"] = runs[starts + within].astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    if total > 64 << 20:
+        raise RuntimeError(f"--dump-outputs: {total} bytes, over the 64 MB bound")
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return {"dir": out_dir, "arrays": len(arrays), "bytes": total}
 
 
 def time_e2e(ctx, batches, paired, steps, D, device):
@@ -630,7 +668,10 @@ def main():
     ap.add_argument("--config-units-scale", type=float, default=1.0)
     ap.add_argument("--cpu-sample-pairs", type=int, default=1_000_000)
     ap.add_argument("--ref-min-seconds", type=float, default=32.0, help="--impl reference: seconds the mapper must run")
-    ap.add_argument("--workdir", default=os.environ.get("URMB_BENCH_DIR", "/dev/shm/urmb_bench"))
+    ap.add_argument("--workdir", default=os.environ.get("URMB_BENCH_DIR"),
+                    help="scratch files (UFI, FASTQ, SAM); default: a new private directory under /dev/shm")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the results of the last timed step (a fixed sample of its reads) to DIR/<name>.npy")
     args = ap.parse_args()
     if args.warmup < 3:
         args.warmup = 3
@@ -649,12 +690,11 @@ def main():
         raise SystemExit("bench.py needs a CUDA device: the mapping engine has no CPU path")
     device = torch.device("cuda", local_rank)
     torch.cuda.set_device(device)
-    from urmap_b200 import build as BLD
-    if rank == 0:
-        BLD.build_engine()
-    if args.impl == "urmb":
-        D.barrier()
     from urmap_b200 import engine
+    from urmap_b200 import build as BLD
+    if not BLD.is_current():   # asks make without building: the tree may be read-only here
+        raise SystemExit("liburmb.so or the CLI is older than its sources: run __graft_entry__.build() first")
+    engine.lib()
 
     baseline = load_json("BASELINE.json")
     peaks = load_json("MEASURED_PEAKS.json")
@@ -674,15 +714,21 @@ def main():
     nb = 3
     B, RL = args.pairs_per_step, args.read_len
     batches = make_batches(meta, seq, device, nb, B, paired, RL, args.sub, args.indel, seed0=1000 * (rank + 1))
-    os.makedirs(args.workdir, exist_ok=True)
+    own_workdir = args.workdir is None
+    if own_workdir:
+        args.workdir = tempfile.mkdtemp(prefix="urmb_bench_", dir="/dev/shm" if os.path.isdir("/dev/shm") else None)
+    else:
+        os.makedirs(args.workdir, exist_ok=True)
+    # scratch files reach tens of GB at human scale (the UFI file) and /dev/shm is RAM: removed however the run ends
+    if (own_workdir or args.workdir.startswith("/dev/shm")) and (own_workdir or rank == 0) \
+            and not os.environ.get("URMB_KEEP_BENCH_DIR"):
+        atexit.register(shutil.rmtree, args.workdir, True)
     ufi_path = os.path.join(args.workdir, "bench.ufi")
     prefix = os.path.join(args.workdir, "sample")
     threads = os.cpu_count()
 
     # ------------------------------------------------------------------ reference arm
     if args.impl == "reference":
-        from oracle import oracle_py as O
-        O.build(ref=True)
         t0 = time.time()
         write_ufi_file(ufi_path, meta, seq, blob)
         log(f"UFI file written for the reference in {time.time() - t0:.1f}s")
@@ -746,8 +792,6 @@ def main():
                 "index_built_by": "urmb_build_index_device on the GPU (byte-identical UFI; setup, not timed)",
                 "load_seconds": r["load_seconds"]}
         print(json.dumps(line), file=_OUT, flush=True)
-        if args.workdir.startswith("/dev/shm") and not os.environ.get("URMB_KEEP_BENCH_DIR"):
-            shutil.rmtree(args.workdir, ignore_errors=True)
         return 0
 
     # ------------------------------------------------------------------ urmb arm
@@ -770,8 +814,10 @@ def main():
     sampler.start()
     sampler.active = True
     # ---- value: inputs resident in HBM, kernels only, CUDA events on the launching stream
-    tv = time_steps(ctx, batches, paired, args.steps, args.warmup, D, device)
+    tv = time_steps(ctx, batches, paired, args.steps, args.warmup, D, device, keep_last=bool(args.dump_outputs))
     sampler.active = False
+    if args.dump_outputs and rank == 0:
+        log(f"outputs of the last timed step: {dump_outputs(args.dump_outputs, tv.pop('last'))}")
     D.barrier()
     kms, klaunch = tv["kernel_ms"], tv["kernel_launches"]
     dev_ms_max = D.max_over_ranks(tv["dev_ms"], device)
@@ -828,8 +874,6 @@ def main():
     cpu_baseline, sam_id, algo, cli = None, None, None, None
     if rank == 0 and world == 1 and not args.no_cpu_baseline:
         try:
-            from oracle import oracle_py as O
-            O.build(ref=True)
             t0 = time.time()
             write_ufi_file(ufi_path, meta, seq, blob)
             log(f"UFI file for the CPU baseline written in {time.time() - t0:.1f}s")
@@ -985,8 +1029,6 @@ def main():
         }
         print(json.dumps(line), file=_OUT, flush=True)
     ctx.close()
-    if args.workdir.startswith("/dev/shm") and rank == 0 and not os.environ.get("URMB_KEEP_BENCH_DIR"):
-        shutil.rmtree(args.workdir, ignore_errors=True)
     D.finalize()
     return 0
 

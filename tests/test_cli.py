@@ -6,7 +6,7 @@ import subprocess
 
 import pytest
 
-from conftest import ROOT, have_gpu
+from conftest import ROOT, expect, file_digest, have_gpu, make_ufi, sam_digest
 from urmap_b200 import synth
 
 BIN = os.path.join(ROOT, "urmap_b200", "bin", "urmap_b200")
@@ -24,21 +24,13 @@ def run(args, **kw):
 
 def test_make_ufi_is_byte_identical(cli, golden_dir, tmp_path):
     """-make_ufi (CPU builder) reproduces the reference's UFI file byte for byte (ufindex.cpp:83-408)."""
-    out = tmp_path / "ref.ufi"
-    r = run([cli, "-make_ufi", os.path.join(golden_dir, "ref.fa"), "-output", str(out), "-quiet"])
-    assert r.returncode == 0, r.stderr
-    assert open(out, "rb").read() == open(os.path.join(golden_dir, "ref.ufi"), "rb").read()
+    make_ufi("golden", os.path.join(golden_dir, "ref.fa"), str(tmp_path / "ref.ufi"))
 
 
-def test_make_ufi_options_match_reference(cli, oracle, golden_dir, tmp_path):
-    if not os.path.exists(oracle.REF_BIN):
-        pytest.skip("reference binary not available")
+def test_make_ufi_options_match_reference(cli, golden_dir, tmp_path):
     fa = os.path.join(golden_dir, "ref.fa")
     for extra in (["-veryfast"], ["-maxix", "5", "-load_factor", "0.7"], ["-slots", "300007"], ["-wordlength", "20"]):
-        a, b = tmp_path / "a.ufi", tmp_path / "b.ufi"
-        assert run([cli, "-make_ufi", fa, "-output", str(a), "-quiet"] + extra).returncode == 0
-        oracle.run_reference(["-make_ufi", fa, "-output", str(b)] + extra)
-        assert open(a, "rb").read() == open(b, "rb").read(), extra
+        make_ufi("golden" + "".join("_" + e.lstrip("-") for e in extra), fa, str(tmp_path / "a.ufi"), extra)
 
 
 def test_invalid_command_lines(cli):
@@ -214,16 +206,14 @@ def test_cli_tabbedout_matches_golden(cli, golden_dir, tmp_path, name, extra):
 
 @pytest.mark.gpu
 def test_cli_tabbedout_repeat_rich_vs_reference(cli, oracle, tmp_path):
-    """Many second pairs: 2 Mb repeat-rich genome, 6 000 pairs (some mates damaged); the reference binary writes the
-    expected file at test time (-threads 1 keeps its output in input order)."""
+    """Many second pairs: 2 Mb repeat-rich genome, 6 000 pairs (some mates damaged); the file equals the reference's
+    (stored digest) and, where the reference binary has been built, the one it writes (-threads 1: input order)."""
     if not have_gpu():
         pytest.skip("no CUDA device")
-    if not os.path.exists(oracle.REF_BIN):
-        pytest.skip("reference binary not available")
     g = synth.make_genome(2_000_000, n_contigs=4, seed=78, repeat_frac=0.15, n_runs=[(2, 0.3, 1500)], tandem=20, segdup=6)
     fa, ufi = str(tmp_path / "ref.fa"), str(tmp_path / "ref.ufi")
     g.write_fasta(fa)
-    oracle.run_reference(["-make_ufi", fa, "-output", ufi])
+    make_ufi("repeat_rich_2mb_seed78", fa, ufi)
     r1, r2, names = synth.sim_pe(g, 6000, 150, 0.02, 0.002, seed=5)
     r2 = r2.copy()
     r2[::40, :75] = r1[::40, :75]
@@ -233,14 +223,16 @@ def test_cli_tabbedout_repeat_rich_vs_reference(cli, oracle, tmp_path):
                 s = arr[i].tobytes()
                 f.write(b"@" + names[i] + b".%d" % i + sfx + b"\n" + s + b"\n+\n" + b"I" * len(s) + b"\n")
     args = ["-map2", str(tmp_path / "r_1.fq"), "-reverse", str(tmp_path / "r_2.fq"), "-ufi", ufi]
-    oracle.run_reference(args + ["-samout", str(tmp_path / "ref.sam"), "-tabbedout", str(tmp_path / "ref.tab"), "-threads", "1"])
     r = run([cli] + args + ["-samout", str(tmp_path / "o.sam"), "-tabbedout", str(tmp_path / "o.tab"), "-batch", "1000"])
     assert r.returncode == 0, r.stderr
-    want = open(tmp_path / "ref.tab", "rb").read().split(b"\n")
     got = open(tmp_path / "o.tab", "rb").read().split(b"\n")
-    assert sum(1 for l in want if l and l.split(b"\t")[3] != b"*") > 100   # the case is exercised
-    diff = [(a, b) for a, b in zip(want, got) if a != b]
-    assert len(want) == len(got) and not diff, diff[:5]
+    assert sum(1 for l in got if l and l.split(b"\t")[3] != b"*") > 100   # the case is exercised
+    expect("tab/repeat_rich_2mb_seed78", file_digest(tmp_path / "o.tab"))
+    if os.path.exists(oracle.REF_BIN):
+        oracle.run_reference(args + ["-samout", str(tmp_path / "ref.sam"), "-tabbedout", str(tmp_path / "ref.tab"), "-threads", "1"])
+        want = open(tmp_path / "ref.tab", "rb").read().split(b"\n")
+        diff = [(a, b) for a, b in zip(want, got) if a != b]
+        assert len(want) == len(got) and not diff, diff[:5]
 
 
 @pytest.mark.gpu
@@ -278,37 +270,52 @@ def test_cli_config1_gate(cli, oracle, tmp_path, contigs):
     """BASELINE.json configs[0] at its stated size: 5 000 000 bp of iid uniform ACGT (one contig, and the three-contig variant
     that exercises the contig padding and SetMappedPos), 100 000 x 150 bp single-end reads with 1 % substitutions and 0.1 %
     indels -- and the same number of read pairs.  The drop-in builds the index on the GPU (byte-identical to the reference's
-    file) and maps from FASTQ files; the reference binary (-threads 1: input order) writes the expected SAM files."""
+    file) and maps from FASTQ files; its SAM files equal the reference's (stored digests), the oracle restatement's, and
+    those of the reference binary (-threads 1: input order) where it has been built."""
     if not have_gpu():
         pytest.skip("no CUDA device")
-    if not os.path.exists(oracle.REF_BIN):
-        pytest.skip("reference binary not available")
     g = synth.make_genome(5_000_000, n_contigs=contigs, seed=12345)
     fa, ufi, mine = str(tmp_path / "ref.fa"), str(tmp_path / "ref.ufi"), str(tmp_path / "mine.ufi")
     g.write_fasta(fa)
-    oracle.run_reference(["-make_ufi", fa, "-output", ufi])
+    make_ufi(f"config1_5mb_{contigs}_contigs", fa, ufi)
     r = run([cli, "-make_ufi", fa, "-output", mine, "-gpu_build", "-quiet"])
     assert r.returncode == 0, r.stderr
     assert open(mine, "rb").read() == open(ufi, "rb").read()
+    ix = oracle.Index(ufi)
     reads, names = synth.sim_se(g, 100_000, 150, 0.01, 0.001, seed=777)
     fq = str(tmp_path / "se.fq")
     synth.write_fastq(fq, reads, names)
-    want, got = str(tmp_path / "ref_se.sam"), str(tmp_path / "se.sam")
-    oracle.run_reference(["-map", fq, "-ufi", ufi, "-samout", want, "-threads", "1"])
+    b = oracle.ReadBatch.from_fastq(fq)
+    res, runs = oracle.map_se(ix, b, threads=os.cpu_count())
+    wants = [oracle.sam_header(ix) + oracle.sam_se(ix, b, res, runs)]
+    got = str(tmp_path / "se.sam")
+    if os.path.exists(oracle.REF_BIN):
+        wants.append(str(tmp_path / "ref_se.sam"))
+        oracle.run_reference(["-map", fq, "-ufi", ufi, "-samout", wants[-1], "-threads", "1"])
     r = run([cli, "-map", fq, "-ufi", mine, "-samout", got, "-quiet"])
     assert r.returncode == 0, r.stderr
-    c = synth.compare_sam(want, got)
-    assert c["identical"] == c["total"] == 100_000 and c["header_equal"], c["diffs"][:5]
+    expect(f"sam/config1_5mb_{contigs}_contigs_se", sam_digest(got))
+    for want in wants:
+        c = synth.compare_sam(want, got)
+        assert c["identical"] == c["total"] == 100_000 and c["header_equal"], c["diffs"][:5]
     r1, r2, names = synth.sim_pe(g, 100_000, 150, 0.01, 0.001, seed=778)
     f1, f2 = str(tmp_path / "p1.fq"), str(tmp_path / "p2.fq")
     synth.write_fastq(f1, r1, names, b"/1")
     synth.write_fastq(f2, r2, names, b"/2")
-    want, got = str(tmp_path / "ref_pe.sam"), str(tmp_path / "pe.sam")
-    oracle.run_reference(["-map2", f1, "-reverse", f2, "-ufi", ufi, "-samout", want, "-threads", "1"])
+    b1, b2 = oracle.ReadBatch.from_fastq(f1), oracle.ReadBatch.from_fastq(f2)
+    o1, o2, runs = oracle.map_pe(ix, b1, b2, threads=os.cpu_count())
+    wants = [oracle.sam_header(ix) + oracle.sam_pe(ix, b1, b2, o1, o2, runs)]
+    got = str(tmp_path / "pe.sam")
+    if os.path.exists(oracle.REF_BIN):
+        wants.append(str(tmp_path / "ref_pe.sam"))
+        oracle.run_reference(["-map2", f1, "-reverse", f2, "-ufi", ufi, "-samout", wants[-1], "-threads", "1"])
     r = run([cli, "-map2", f1, "-reverse", f2, "-ufi", mine, "-samout", got, "-quiet"])
     assert r.returncode == 0, r.stderr
-    c = synth.compare_sam(want, got)
-    assert c["identical"] == c["total"] == 200_000 and c["header_equal"], c["diffs"][:5]
+    expect(f"sam/config1_5mb_{contigs}_contigs_pe", sam_digest(got))
+    for want in wants:
+        c = synth.compare_sam(want, got)
+        assert c["identical"] == c["total"] == 200_000 and c["header_equal"], c["diffs"][:5]
+    ix.close()
 
 
 @pytest.mark.gpu
@@ -316,16 +323,14 @@ def test_cli_contig_end_overhang(cli, oracle, tmp_path):
     """Pairs with a mate hanging 1 - 10 bases over either end of a contig: State1::SetMappedPos (state1.cpp:129-145) clears
     the top hit of such a mate, and OutputTab2 sees that cleared state only when a SAM file is written first
     (output2.cpp:10-16): the -tabbedout file differs with and without -samout.  Both forms, and the SAM file, equal the
-    reference binary's."""
+    reference's (stored digests) and, where the reference binary has been built, the files it writes."""
     if not have_gpu():
         pytest.skip("no CUDA device")
-    if not os.path.exists(oracle.REF_BIN):
-        pytest.skip("reference binary not available")
     import numpy as np
     g = synth.make_genome(600_000, n_contigs=3, seed=99)
     fa, ufi = str(tmp_path / "ref.fa"), str(tmp_path / "ref.ufi")
     g.write_fasta(fa)
-    oracle.run_reference(["-make_ufi", fa, "-output", ufi])
+    make_ufi("overhang_600kb_seed99", fa, ufi)
     rng = np.random.default_rng(5)
     comp = np.zeros(256, np.uint8)
     for a, b in zip(b"ACGT", b"TGCA"):
@@ -354,17 +359,22 @@ def test_cli_contig_end_overhang(cli, oracle, tmp_path):
     synth.write_fastq(f2, np.array(r2), names, b"/2")
     args = ["-map2", f1, "-reverse", f2, "-ufi", ufi]
     p = lambda n: str(tmp_path / n)
-    oracle.run_reference(args + ["-threads", "1", "-samout", p("ref.sam"), "-tabbedout", p("ref_a.tab")])
-    oracle.run_reference(args + ["-threads", "1", "-tabbedout", p("ref_b.tab")])
-    assert open(p("ref_a.tab"), "rb").read() != open(p("ref_b.tab"), "rb").read()   # the case is what it claims to be
     r = run([cli] + args + ["-samout", p("o.sam"), "-tabbedout", p("o_a.tab"), "-batch", "16", "-quiet"])
     assert r.returncode == 0, r.stderr
     r = run([cli] + args + ["-tabbedout", p("o_b.tab"), "-batch", "16", "-quiet"])
     assert r.returncode == 0, r.stderr
-    assert open(p("o_a.tab"), "rb").read() == open(p("ref_a.tab"), "rb").read()
-    assert open(p("o_b.tab"), "rb").read() == open(p("ref_b.tab"), "rb").read()
-    c = synth.compare_sam(p("ref.sam"), p("o.sam"))
-    assert c["identical"] == c["total"] == 2 * len(names) and c["header_equal"], c["diffs"][:5]
+    assert open(p("o_a.tab"), "rb").read() != open(p("o_b.tab"), "rb").read()   # the case is what it claims to be
+    expect("tab/overhang_600kb_seed99_with_samout", file_digest(p("o_a.tab")))
+    expect("tab/overhang_600kb_seed99_without_samout", file_digest(p("o_b.tab")))
+    expect("sam/overhang_600kb_seed99", sam_digest(p("o.sam")))
+    assert sam_digest(p("o.sam"))["records"] == 2 * len(names)
+    if os.path.exists(oracle.REF_BIN):
+        oracle.run_reference(args + ["-threads", "1", "-samout", p("ref.sam"), "-tabbedout", p("ref_a.tab")])
+        oracle.run_reference(args + ["-threads", "1", "-tabbedout", p("ref_b.tab")])
+        assert open(p("o_a.tab"), "rb").read() == open(p("ref_a.tab"), "rb").read()
+        assert open(p("o_b.tab"), "rb").read() == open(p("ref_b.tab"), "rb").read()
+        c = synth.compare_sam(p("ref.sam"), p("o.sam"))
+        assert c["identical"] == c["total"] == 2 * len(names) and c["header_equal"], c["diffs"][:5]
 
 
 def test_ufi_validate(cli, oracle, golden_dir, tmp_path):
@@ -425,9 +435,7 @@ def _unused(stderr):
 def test_unused_option_warnings(cli, oracle, golden_dir, tmp_path, cmd):
     """CheckUsedOpts (cmdline.cpp:13-26): an option that was given but that the command never looks at is named in a warning
     after the command has run, in the order of myopts.h -- the same names in the same order as the reference binary prints
-    (this program uses -threads for -ufi_validate, the one deliberate difference)."""
-    if not os.path.exists(oracle.REF_BIN):
-        pytest.skip("reference binary not available")
+    (this program uses -threads for -ufi_validate, the one deliberate difference).  The reference's names are stored."""
     import subprocess
     g = golden_dir
     base = {"make_ufi": ["-make_ufi", os.path.join(g, "ref.fa"), "-output", str(tmp_path / "o.ufi")],
@@ -437,13 +445,18 @@ def test_unused_option_warnings(cli, oracle, golden_dir, tmp_path, cmd):
               "-load_factor", "0.6", "-wordlength", "24", "-ufi", os.path.join(g, "ref.ufi"), "-samout", str(tmp_path / "x.sam")]
     if cmd == "make_ufi":
         extras = [e for e in extras if e not in ("-maxix", "32", "-wordlength", "24", "-load_factor", "0.6", "-validate")] + ["-validate"]
-    ref = subprocess.run([oracle.REF_BIN] + base + extras, capture_output=True, text=True)
     mine = run([cli] + base + extras)
-    assert ref.returncode == 0 and mine.returncode == 0, (ref.stderr[-300:], mine.stderr[-300:])
-    want = _unused(ref.stderr)
-    if cmd == "ufi_validate":
-        want = [w for w in want if w != "threads"]
-    assert _unused(mine.stderr) == want and len(want) >= 3
+    assert mine.returncode == 0, mine.stderr[-300:]
+    got = _unused(mine.stderr)
+    expect("unused_options/" + cmd, got)   # for -ufi_validate: the reference's names but -threads
+    if os.path.exists(oracle.REF_BIN):
+        ref = subprocess.run([oracle.REF_BIN] + base + extras, capture_output=True, text=True)
+        assert ref.returncode == 0, ref.stderr[-300:]
+        want = _unused(ref.stderr)
+        if cmd == "ufi_validate":
+            want = [w for w in want if w != "threads"]
+        assert got == want
+    assert len(got) >= 3
 
 
 @pytest.mark.gpu

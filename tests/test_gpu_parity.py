@@ -6,7 +6,7 @@ import os
 import numpy as np
 import pytest
 
-from conftest import ROOT, have_gpu
+from conftest import CLI, have_gpu, make_ufi
 from urmap_b200 import synth
 
 pytestmark = pytest.mark.gpu
@@ -77,14 +77,12 @@ def test_golden_pe(eng, oracle, golden_oix, golden_dir, golden_ctxs, key):
 
 @pytest.fixture(scope="module")
 def mid_env(eng, oracle, tmp_path_factory):
-    """2 Mb repeat-rich reference indexed by the reference binary (travels in oracle/_ref/)."""
-    if not os.path.exists(oracle.REF_BIN):
-        pytest.skip("reference binary not available to build the index")
+    """2 Mb repeat-rich reference indexed by the host builder."""
     d = tmp_path_factory.mktemp("mid")
     g = synth.make_genome(2_000_000, n_contigs=4, seed=77, repeat_frac=0.10, n_runs=[(2, 0.3, 1500)], tandem=20, segdup=4)
     fa, ufi = str(d / "ref.fa"), str(d / "ref.ufi")
     g.write_fasta(fa)
-    oracle.run_reference(["-make_ufi", fa, "-output", ufi])
+    make_ufi("mid_2mb_seed77", fa, ufi)
     return g, oracle.Index(ufi), eng.HostIndex(ufi)
 
 
@@ -247,15 +245,13 @@ def test_chunk_size_invariance(eng, oracle, mid_env):
 
 
 def test_dense_index_long_links(eng, oracle, tmp_path):
-    """Mapping parity on an index full of long links (tallies 125 / 253, ufindex.cpp:256-300, 905-926): the reference
-    binary builds the 2 Mb repeat-rich genome at load factor 0.95 (tens of thousands of long-link records); single-end
+    """Mapping parity on an index full of long links (tallies 125 / 253, ufindex.cpp:256-300, 905-926): the host
+    builder indexes the 2 Mb repeat-rich genome at load factor 0.95 (tens of thousands of long-link records); single-end
     (rows of both row kernels walk them) and paired-end results equal the oracle's on the same index."""
-    if not os.path.exists(oracle.REF_BIN):
-        pytest.skip("reference binary not available to build the index")
     g = synth.make_genome(2_000_000, n_contigs=4, seed=77, repeat_frac=0.10, n_runs=[(2, 0.3, 1500)], tandem=20, segdup=4)
     fa, ufi = str(tmp_path / "ref.fa"), str(tmp_path / "dense.ufi")
     g.write_fasta(fa)
-    oracle.run_reference(["-make_ufi", fa, "-output", ufi, "-load_factor", "0.95"])
+    make_ufi("mid_2mb_seed77_load_factor_0.95", fa, ufi, ["-load_factor", "0.95"])
     oix, hix = oracle.Index(ufi), eng.HostIndex(ufi)
     tallies = oix.blob()[0::5]
     assert int(((tallies == 125) | (tallies == 253)).sum()) > 10000
@@ -276,17 +272,15 @@ def test_dense_index_long_links(eng, oracle, tmp_path):
 
 
 def test_maxix_above_32(eng, oracle, tmp_path):
-    """An index built with -maxix 100 (ufindexio.cpp:135-136) by the drop-in's GPU builder: byte-identical to the reference's,
-    and rows of 33 .. 100 positions (tandem arrays) are mapped as the oracle maps them, single-end and paired."""
-    if not os.path.exists(oracle.REF_BIN):
-        pytest.skip("reference binary not available to build the index")
+    """An index built with -maxix 100 (ufindexio.cpp:135-136) by the drop-in's GPU builder: byte-identical to the host
+    builder's (and so to the reference's), and rows of 33 .. 100 positions (tandem arrays) are mapped as the oracle maps
+    them, single-end and paired."""
     import subprocess
     g = synth.make_genome(1_000_000, n_contigs=3, seed=78, repeat_frac=0.30, n_runs=[(0, 0.3, 300)], tandem=40)
     fa, ufi, mine = str(tmp_path / "m.fa"), str(tmp_path / "m.ufi"), str(tmp_path / "mine.ufi")
     g.write_fasta(fa)
-    oracle.run_reference(["-make_ufi", fa, "-output", ufi, "-maxix", "100"])
-    cli = os.path.join(ROOT, "urmap_b200", "bin", "urmap_b200")
-    r = subprocess.run([cli, "-make_ufi", fa, "-output", mine, "-maxix", "100", "-gpu_build", "-quiet"], capture_output=True, text=True)
+    make_ufi("m_1mb_seed78_maxix_100", fa, ufi, ["-maxix", "100"])
+    r = subprocess.run([CLI, "-make_ufi", fa, "-output", mine, "-maxix", "100", "-gpu_build", "-quiet"], capture_output=True, text=True)
     assert r.returncode == 0, r.stderr
     assert open(mine, "rb").read() == open(ufi, "rb").read()
     oix, hix = oracle.Index(ufi), eng.HostIndex(mine)

@@ -1,22 +1,31 @@
-"""Pins the oracle restatement against the UNMODIFIED reference binary (oracle/_ref/urmap) on fresh seeded data.
-Skipped where the binary is absent (it is built from /root/reference/src by oracle/Makefile when that exists)."""
+"""Pins the oracle restatement against the UNMODIFIED reference binary on fresh seeded data: its SAM files equal the
+reference's (stored digests, tests/golden/reference_outputs.json) and, where the binary has been built (oracle/_ref/urmap,
+from the reference's sources by oracle/Makefile), the files it writes at test time."""
 import os
 
 import pytest
 
+from conftest import expect, make_ufi, sam_digest
 from urmap_b200 import synth
 
 
 @pytest.fixture(scope="module")
-def ref_env(oracle, tmp_path_factory):
-    if not os.path.exists(oracle.REF_BIN):
-        pytest.skip("reference binary not built (no /root/reference here)")
+def ref_env(oracle, built_lib, tmp_path_factory):
     d = tmp_path_factory.mktemp("refenv")
     g = synth.make_genome(1_000_000, n_contigs=2, seed=31, repeat_frac=0.05, n_runs=[(0, 0.3, 500)], tandem=4)
     fa, ufi = str(d / "ref.fa"), str(d / "ref.ufi")
     g.write_fasta(fa)
-    oracle.run_reference(["-make_ufi", fa, "-output", ufi])
+    make_ufi("ovr_1mb_seed31", fa, ufi)
     return d, g, ufi
+
+
+def _check(oracle, key, mine, ref_args, sam, n):
+    assert sam_digest(mine)["records"] == n
+    expect("sam/" + key, sam_digest(mine))
+    if os.path.exists(oracle.REF_BIN):
+        oracle.run_reference(ref_args + ["-samout", sam, "-threads", "1"])
+        c = synth.compare_sam(sam, mine)
+        assert c["identical"] == c["total"] == n and c["header_equal"], c["diffs"][:5]
 
 
 @pytest.mark.parametrize("sub,indel,veryfast", [(0.01, 0.001, False), (0.05, 0.01, False), (0.02, 0.002, True)])
@@ -25,13 +34,12 @@ def test_se_matches_reference(oracle, ref_env, sub, indel, veryfast):
     reads, names = synth.sim_se(g, 4000, 150, sub, indel, seed=int(sub * 1000) + 5)
     fq, sam = str(d / "se.fq"), str(d / "se.sam")
     synth.write_fastq(fq, reads, names)
-    oracle.run_reference(["-map", fq, "-ufi", ufi, "-samout", sam, "-threads", "1"] + (["-veryfast"] if veryfast else []))
     ix = oracle.Index(ufi)
     b = oracle.ReadBatch.from_fastq(fq)
     res, runs = oracle.map_se(ix, b, method=7 if veryfast else 6, threads=4)
     mine = oracle.sam_header(ix) + oracle.sam_se(ix, b, res, runs)
-    c = synth.compare_sam(sam, mine)
-    assert c["identical"] == c["total"] == 4000 and c["header_equal"], c["diffs"][:5]
+    _check(oracle, f"ovr_se_{sub}_{indel}{'_veryfast' if veryfast else ''}", mine,
+           ["-map", fq, "-ufi", ufi] + (["-veryfast"] if veryfast else []), sam, 4000)
 
 
 @pytest.mark.parametrize("sub,indel,veryfast,rl", [(0.01, 0.001, False, 150), (0.05, 0.01, False, 150), (0.02, 0.002, True, 150),
@@ -42,42 +50,36 @@ def test_pe_matches_reference(oracle, ref_env, sub, indel, veryfast, rl):
     f1, f2, sam = str(d / "p1.fq"), str(d / "p2.fq"), str(d / "pe.sam")
     synth.write_fastq(f1, r1, names, b"/1")
     synth.write_fastq(f2, r2, names, b"/2")
-    oracle.run_reference(["-map2", f1, "-reverse", f2, "-ufi", ufi, "-samout", sam, "-threads", "1"]
-                         + (["-veryfast"] if veryfast else []))
     ix = oracle.Index(ufi)
     b1, b2 = oracle.ReadBatch.from_fastq(f1), oracle.ReadBatch.from_fastq(f2)
     o1, o2, runs = oracle.map_pe(ix, b1, b2, pe_method=5 if veryfast else 4, threads=4)
     mine = oracle.sam_header(ix) + oracle.sam_pe(ix, b1, b2, o1, o2, runs)
-    c = synth.compare_sam(sam, mine)
-    assert c["identical"] == c["total"] == 6000 and c["header_equal"], c["diffs"][:5]
+    _check(oracle, f"ovr_pe_{rl}_{sub}_{indel}{'_veryfast' if veryfast else ''}", mine,
+           ["-map2", f1, "-reverse", f2, "-ufi", ufi] + (["-veryfast"] if veryfast else []), sam, 6000)
 
 
-def test_maxix_above_32_matches_reference(oracle, tmp_path):
+def test_maxix_above_32_matches_reference(oracle, built_lib, tmp_path):
     """-maxix 100 (ufindexio.cpp:135-136): the reference indexes and walks lists of up to 100 positions; the restatement's
     rows follow (repeat-rich genome with tandem arrays, single-end and paired)."""
-    if not os.path.exists(oracle.REF_BIN):
-        pytest.skip("reference binary not built (no /root/reference here)")
     g = synth.make_genome(300_000, n_contigs=2, seed=78, repeat_frac=0.35, n_runs=[(0, 0.3, 300)], tandem=12)
     fa, ufi = str(tmp_path / "m.fa"), str(tmp_path / "m.ufi")
     g.write_fasta(fa)
-    oracle.run_reference(["-make_ufi", fa, "-output", ufi, "-maxix", "100"])
+    make_ufi("ovr_300kb_seed78_maxix_100", fa, ufi, ["-maxix", "100"])
     ix = oracle.Index(ufi)
     assert ix.max_ix == 100
     reads, names = synth.sim_se(g, 1500, 150, 0.02, 0.002, seed=5)
     fq, sam = str(tmp_path / "se.fq"), str(tmp_path / "se.sam")
     synth.write_fastq(fq, reads, names)
-    oracle.run_reference(["-map", fq, "-ufi", ufi, "-samout", sam, "-threads", "1"])
     b = oracle.ReadBatch.from_fastq(fq)
     res, runs = oracle.map_se(ix, b, threads=4)
-    c = synth.compare_sam(sam, oracle.sam_header(ix) + oracle.sam_se(ix, b, res, runs))
-    assert c["identical"] == c["total"] == 1500 and c["header_equal"], c["diffs"][:5]
+    _check(oracle, "ovr_maxix_100_se", oracle.sam_header(ix) + oracle.sam_se(ix, b, res, runs), ["-map", fq, "-ufi", ufi],
+           sam, 1500)
     r1, r2, names = synth.sim_pe(g, 1000, 150, 0.02, 0.002, seed=15)
     f1, f2, sam2 = str(tmp_path / "p1.fq"), str(tmp_path / "p2.fq"), str(tmp_path / "pe.sam")
     synth.write_fastq(f1, r1, names, b"/1")
     synth.write_fastq(f2, r2, names, b"/2")
-    oracle.run_reference(["-map2", f1, "-reverse", f2, "-ufi", ufi, "-samout", sam2, "-threads", "1"])
     b1, b2 = oracle.ReadBatch.from_fastq(f1), oracle.ReadBatch.from_fastq(f2)
     o1, o2, runs = oracle.map_pe(ix, b1, b2, threads=4)
-    c = synth.compare_sam(sam2, oracle.sam_header(ix) + oracle.sam_pe(ix, b1, b2, o1, o2, runs))
-    assert c["identical"] == c["total"] == 2000 and c["header_equal"], c["diffs"][:5]
+    _check(oracle, "ovr_maxix_100_pe", oracle.sam_header(ix) + oracle.sam_pe(ix, b1, b2, o1, o2, runs),
+           ["-map2", f1, "-reverse", f2, "-ufi", ufi], sam2, 2000)
     ix.close()

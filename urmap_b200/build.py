@@ -15,6 +15,11 @@ def _stale(target, sources):
     return any(os.path.getmtime(s) > t for s in sources if os.path.exists(s))
 
 
+def is_current():
+    """True when liburmb.so and the host tools are up to date with their sources (make -q: nothing is built)."""
+    return subprocess.call(["make", "-q", "-C", CSRC], stdout=subprocess.DEVNULL, stderr=subprocess.DEVNULL) == 0
+
+
 def build_engine(force=False, verbose=False):
     """nvcc -gencode arch=compute_100a,code=sm_100a -lineinfo ... -> urmap_b200/liburmb.so (+ bin/urmap_b200)."""
     out = None if verbose else subprocess.DEVNULL
