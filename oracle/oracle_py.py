@@ -73,6 +73,8 @@ def lib():
         L.uo_revcomp.argtypes = [vp, C.c_uint32, vp]
         L.uo_viterbi.restype = C.c_float
         L.uo_viterbi.argtypes = [C.POINTER(Params), vp, C.c_uint32, vp, C.c_uint32, C.c_int, C.c_int, C.c_char_p]
+        L.uo_viterbi_ex.restype = C.c_float
+        L.uo_viterbi_ex.argtypes = [C.POINTER(Params), vp, C.c_uint32, vp, C.c_uint32, C.c_int, C.c_int, C.c_char_p, vp]
         L.uo_path_to_cigar.argtypes = [C.c_char_p, C.c_uint32, C.c_char_p]
         L.uo_index_functional_diff.restype = C.c_uint64
         L.uo_index_functional_diff.argtypes = [vp, vp, vp]
@@ -240,6 +242,19 @@ def viterbi(A: bytes, B: bytes, left: bool, right: bool, method=6, band_radius=-
     sc = lib().uo_viterbi(C.byref(p), _p(a) if len(a) else None, len(a), _p(b) if len(b) else None, len(b),
                           int(left), int(right), buf)
     return float(sc), buf.value.decode()
+
+
+def viterbi_ex(A: bytes, B: bytes, left: bool, right: bool, method=6, band_radius=-1):
+    """viterbi() plus the number of traceback reads of cells the call never wrote (the result is undefined when it is
+    not zero): (score, path, poison reads)."""
+    p = Params(method, 4, band_radius, 10)
+    buf = C.create_string_buffer(len(A) + len(B) + 4)
+    a = np.frombuffer(A, dtype=np.uint8)
+    b = np.frombuffer(B, dtype=np.uint8)
+    n = C.c_uint64(0)
+    sc = lib().uo_viterbi_ex(C.byref(p), _p(a) if len(a) else None, len(a), _p(b) if len(b) else None, len(b),
+                             int(left), int(right), buf, C.addressof(n))
+    return float(sc), buf.value.decode(), int(n.value)
 
 
 def path_to_cigar(path: str, ql: int):

@@ -1536,6 +1536,17 @@ float uo_viterbi(const uo_params *p, const uint8_t *A, uint32_t LA, const uint8_
     return sc;
 }
 
+float uo_viterbi_ex(const uo_params *p, const uint8_t *A, uint32_t LA, const uint8_t *B, uint32_t LB, int left,
+                    int right, char *path, uint64_t *tb_poison_reads) {
+    Params P = MakeParams(p);
+    std::string s;
+    uo_stats st{};
+    float sc = Viterbi(P, A, LA, B, LB, left != 0, right != 0, s, &st);
+    memcpy(path, s.c_str(), s.size() + 1);
+    *tb_poison_reads = st.tb_poison_reads;
+    return sc;
+}
+
 void uo_path_to_cigar(const char *path, uint32_t QL, char *out) {
     std::vector<uint16_t> runs;
     PathToRuns(path, runs);

@@ -99,6 +99,10 @@ void uo_revcomp(const uint8_t *seq, uint32_t L, uint8_t *out);
 /* returns score; path (NUL-terminated, reference path alphabet) must hold LA+LB+2 bytes */
 float uo_viterbi(const uo_params *p, const uint8_t *A, uint32_t LA, const uint8_t *B, uint32_t LB,
                  int left, int right, char *path);
+/* uo_viterbi plus the number of traceback reads of cells the call never wrote (uo_stats::tb_poison_reads): where it
+ * is not zero the reference reads stale bytes there and its result is undefined */
+float uo_viterbi_ex(const uo_params *p, const uint8_t *A, uint32_t LA, const uint8_t *B, uint32_t LB,
+                    int left, int right, char *path, uint64_t *tb_poison_reads);
 /* path -> CIGAR incl. the dangling-M polish (cigar.cpp:4,141); out must hold 12*strlen(path)+16 */
 void uo_path_to_cigar(const char *path, uint32_t QL, char *out);
 uint64_t uo_get_prime(uint64_t n);

@@ -2,7 +2,7 @@
 // Compiles urmap_b200/csrc/urmb_kernels.cu as C++ on top of a lock-step fiber emulation of one warp.
 #include "cuda_runtime.h"
 
-#include "../../urmap_b200/csrc/urmb_kernels.cu"
+#include "../kunit/kunit_cases.cuh"   // urmb_kernels.cu and the single-case runners of tests/kunit
 #include "../../urmap_b200/csrc/urmb_build.cu"
 
 emu_dim3 threadIdx, blockIdx, blockDim, gridDim;
@@ -115,15 +115,9 @@ void launch(const std::function<void()> &body, int grid, int block, size_t smem)
 using namespace urmb;
 
 static DevParams emu_make_params(const urmb_params &p) {  // same table as urmb_api.cu make_params
-    DevParams P;
-    if (p.method == 7) P = DevParams{-4, -6, -2, 35, 35, 12, 75, 8, 6, 5, 8u, 4, 3u};
-    else P = DevParams{-3, -5, -1, 20, 60, 9, 100, 1, 1, 1, 12u, 4, 3u};
-    P.pe_method = (p.pe_method == 5) ? 5 : 4;
-    if (p.band_radius >= 0) P.R = (uint32_t)p.band_radius;
-    else if (p.pe_method == 5) P.R = 4;
-    P.flags = 0;
-    if (const char *f = getenv("URMB_FLAGS")) P.flags = (uint32_t)strtoul(f, nullptr, 0);
-    P.rescue_rounds = 0;
+    uint32_t flags = 0;
+    if (const char *f = getenv("URMB_FLAGS")) flags = (uint32_t)strtoul(f, nullptr, 0);
+    DevParams P = kunit::params(p.method, p.pe_method, p.band_radius, flags);
     if (const char *f = getenv("URMB_RESCUE_ROUNDS")) P.rescue_rounds = std::min(std::max(atoi(f), 0), (int)kRescueRounds);
     return P;
 }
@@ -143,7 +137,7 @@ extern "C" int emu_map(const uint8_t *blob, const uint8_t *seq_padded, uint32_t 
     ix.blob = blob;
     ix.seq = seq_padded;
     ix.slot_count = slot_count;
-    ix.magic = (uint64_t)((((unsigned __int128)1) << 64) / slot_count);
+    ix.magic = barrett_magic(slot_count);
     ix.shift_mask = (word_len >= 32) ? ~0ull : ((1ull << (2 * word_len)) - 1);
     ix.seq_size = seq_size;
     ix.word_len = word_len;
@@ -251,7 +245,7 @@ extern "C" int emu_build_index(const uint8_t *seq, uint64_t seq_size, uint64_t s
     a.seq = seq;
     a.seq_size = seq_size;
     a.slot_count = slot_count;
-    a.magic = (uint64_t)((((unsigned __int128)1) << 64) / slot_count);
+    a.magic = barrett_magic(slot_count);
     a.shift_mask = (word_len >= 32) ? ~0ull : ((1ull << (2 * word_len)) - 1);
     a.word_len = word_len;
     a.max_ix = max_ix;

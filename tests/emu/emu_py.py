@@ -24,7 +24,8 @@ def lib():
     if _lib is None:
         so = os.path.join(HERE, "libemu.so")
         src = [os.path.join(HERE, "emu.cpp"), os.path.join(HERE, "cuda_runtime.h"),
-               os.path.join(HERE, "../../urmap_b200/csrc/urmb_kernels.cu")]
+               os.path.join(HERE, "../../urmap_b200/csrc/urmb_kernels.cu"),
+               os.path.join(HERE, "../../urmap_b200/csrc/urmb_internal.h"), os.path.join(HERE, "../kunit/kunit_cases.cuh")]
         if not os.path.exists(so) or any(os.path.getmtime(s) > os.path.getmtime(so) for s in src):
             subprocess.check_call([os.path.join(HERE, "build.sh")])
         _lib = C.CDLL(so)

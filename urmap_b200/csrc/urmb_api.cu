@@ -398,7 +398,7 @@ static int set_index(urmb_ctx *c, const urmb_index_desc *d) {
     c->ix.blob = (const uint8_t *)d->d_blob;
     c->ix.seq = (const uint8_t *)d->d_seq;
     c->ix.slot_count = d->slot_count;
-    c->ix.magic = (uint64_t)((((unsigned __int128)1) << 64) / d->slot_count);
+    c->ix.magic = barrett_magic(d->slot_count);
     c->ix.shift_mask = (d->word_length >= 32) ? ~0ull : ((1ull << (2 * d->word_length)) - 1);
     c->ix.seq_size = d->seq_data_size;
     c->ix.word_len = d->word_length;

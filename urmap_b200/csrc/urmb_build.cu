@@ -563,7 +563,7 @@ extern "C" int urmb_build_index_device(const void *d_seq, uint64_t seq_data_size
     a.seq = (const uint8_t *)d_seq;
     a.seq_size = seq_data_size;
     a.slot_count = slot_count;
-    a.magic = (uint64_t)((((unsigned __int128)1) << 64) / slot_count);
+    a.magic = barrett_magic(slot_count);
     a.shift_mask = (word_length >= 32) ? ~0ull : ((1ull << (2 * word_length)) - 1);
     a.word_len = word_length;
     a.max_ix = max_ix;

@@ -44,6 +44,9 @@ struct DevIndex {
     uint32_t max_ix;
 };
 
+// floor(2^64 / p), the multiplier of the Barrett reduction h % p (mod_slots; DevIndex::magic)
+inline uint64_t barrett_magic(uint64_t p) { return (uint64_t)((((unsigned __int128)1) << 64) / p); }
+
 struct DevParams {  // State1::SetMethod constants, state1.cpp:147-183
     int MM, GO, GE, MIN_HSP_PCT, TERM3_PCT, XDROP, MAXPEN, XP1, XP3, XP4;
     uint32_t R;
