@@ -194,6 +194,23 @@ int urmb_build_index_device(const void *d_seq, uint64_t seq_data_size, uint64_t 
                             uint32_t max_ix, void *d_blob, uint64_t *stats);
 const char *urmb_build_last_error(void);
 
+/* Index of a FASTA file built on the device(s) of n contexts: the table `-make_ufi` writes for the same word length,
+ * max_ix and slot count, without a file.  fa: the raw (decompressed) FASTA bytes on the host.  *header receives the
+ * contig table (labels, lengths, offsets); its blob / seq pointers are NULL.  The contexts own the device buffers.
+ * The bytes are parsed on every device (urmb_fasta.cu) into exactly the SeqData of UfiBuilder::ReadFasta (urmb_host.cpp,
+ * fastaseqsource.cpp:26-112).  Errors: URMB_E_IO for a bad FASTA ("expected '>' in line N", as -make_ufi) or one without
+ * sequence; URMB_E_UNSUPPORTED for a genome larger than SeqData can address; the builder's own code and message when it
+ * refuses the table (URMB_E_OVERFLOW: a list the reference would truncate, a full repair list; URMB_E_UNSUPPORTED: max_ix
+ * above 254) -- `-make_ufi` builds those tables on the host. */
+int urmb_index_from_fasta(urmb_ctx **ctxs, int n, const uint8_t *fa, uint64_t fa_len, uint32_t word_length,
+                          uint32_t max_ix, uint64_t slot_count, urmb_index_host **header);
+/* Labels of the FASTA records that had no sequence and were dropped (for the warnings -make_ufi prints); URMB_E_ARG past the
+ * last one. */
+int urmb_index_dropped(const urmb_index_host *h, uint32_t i, const char **label);
+/* Seconds spent by urmb_index_from_fasta (host clock around device work that ends in a synchronise; the slowest GPU):
+ * t[0] upload of the raw bytes, t[1] parse, t[2] table build, t[3] packed genome, t[4] device time of the parse kernels. */
+int urmb_index_fasta_times(const urmb_index_host *h, double t[5]);
+
 /* Optional: size all slots for batches of n_units reads (pairs when paired != 0) of up to max_read_len bases ahead of
  * the first urmb_submit.  It touches the slots only and may run on another thread while urmb_index_upload /
  * urmb_index_broadcast of the same context is still copying; word_length is the index's (UFI header). */

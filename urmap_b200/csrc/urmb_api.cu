@@ -55,6 +55,9 @@ struct urmb_index_host {
     std::vector<uint32_t> lengths, offsets;
     const uint8_t *blob = nullptr;
     const uint8_t *seq = nullptr;
+    // urmb_index_from_fasta: header only (blob / seq null), the labels of the dropped records and the times of the steps
+    std::vector<std::string> dropped;
+    double fasta_times[5] = {0, 0, 0, 0, 0};
 };
 
 extern "C" int urmb_index_load_host(const char *path, urmb_index_host **out) {
@@ -562,6 +565,122 @@ extern "C" int urmb_index_broadcast(urmb_ctx **ctxs, int n, const urmb_index_hos
         });
     for (auto &t : th) t.join();
     for (int i = 0; i < n; ++i) if (rcs[i]) return rcs[i];
+    return URMB_OK;
+}
+
+// Index of a FASTA file built on the devices of n contexts (no UFI file): the raw bytes go to every GPU through the
+// fan-out of upload_region (3.1 GB for a human genome instead of the 30 GB table), then each GPU parses them
+// (urmb_fasta.cu), frees them, builds the table (urmb_build_index_device) and derives its packed genome on its own host
+// thread, all at the same time.
+extern "C" int urmb_index_from_fasta(urmb_ctx **ctxs, int n, const uint8_t *fa, uint64_t fa_len, uint32_t word_length,
+                                     uint32_t max_ix, uint64_t slot_count, urmb_index_host **header) {
+    if (!ctxs || n < 1 || !header || (!fa && fa_len)) return URMB_E_ARG;
+    *header = nullptr;
+    for (int i = 0; i < n; ++i) if (!ctxs[i]) return URMB_E_ARG;
+    urmb_ctx *c = ctxs[0];
+    if (slot_count < 2) return fail(c, URMB_E_ARG, "bad slot count");
+    auto now = []() { return std::chrono::duration<double>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
+    const double t0 = now();
+    const uint64_t padded = fasta_padded_len(fa_len);
+    std::vector<void *> d_fa(n, nullptr);
+    struct Release {   // the raw bytes, on every return
+        std::vector<urmb_ctx *> ctxs; std::vector<void *> *d_fa;
+        ~Release() { for (size_t i = 0; i < ctxs.size(); ++i) if ((*d_fa)[i]) { cudaSetDevice(ctxs[i]->device); cudaFree((*d_fa)[i]); } }
+    } release{std::vector<urmb_ctx *>(ctxs, ctxs + n), &d_fa};
+    Fanout fan;
+    fan.n = n;
+    fan.ctxs = ctxs;
+    fan.dst.assign(n, nullptr);
+    fan.streams.assign(n, nullptr);
+    for (int i = 0; i < n; ++i) {
+        urmb_ctx *c = ctxs[i];   // errors below are reported against the context they belong to
+        CK(cudaSetDevice(c->device));
+        c->have_index = false;
+        cudaFree(c->own_blob);
+        cudaFree(c->own_seq);
+        c->own_blob = c->own_seq = nullptr;
+        CK(cudaMalloc(&d_fa[i], padded));
+        CK(cudaMemset((uint8_t *)d_fa[i] + fa_len, 0, padded - fa_len));
+        if (i > 0) {
+            int can = 0;
+            cudaDeviceCanAccessPeer(&can, c->device, ctxs[0]->device);
+            if (can) cudaDeviceEnablePeerAccess(ctxs[0]->device, 0);
+            cudaGetLastError();
+        }
+        fan.dst[i] = d_fa[i];
+        fan.streams[i] = c->slots[0].copy;
+    }
+    int rc = upload_region(c, d_fa[0], fa, fa_len, &fan);
+    if (rc) return rc;
+    const double t1 = now();
+    std::vector<int> rcs(n, 0);
+    std::vector<FastaTable> tabs(n);
+    std::vector<double> t_parse(n, 0), t_build(n, 0), t_pack(n, 0);
+    std::vector<float> k_ms(n, 0);
+    std::vector<std::thread> th;
+    for (int i = 0; i < n; ++i)
+        th.emplace_back([&, i]() {
+            urmb_ctx *c = ctxs[i];
+            rcs[i] = [&]() -> int {
+                CK(cudaSetDevice(c->device));
+                const double a = now();
+                void *d_seq = nullptr;
+                std::string err;
+                int r = fasta_parse_device((const uint8_t *)d_fa[i], fa, fa_len, c->compute, &d_seq, tabs[i], &k_ms[i], err);
+                cudaFree(d_fa[i]);   // before the build: the raw bytes are not needed any more
+                d_fa[i] = nullptr;
+                if (r) return fail(c, r, err);
+                c->own_seq = d_seq;
+                const double b = now();
+                t_parse[i] = b - a;
+                const uint64_t nb = 5 * slot_count;
+                CK(cudaMalloc(&c->own_blob, nb + URMB_BLOB_PAD));
+                uint64_t stats[3] = {0, 0, 0};
+                r = urmb_build_index_device(c->own_seq, tabs[i].seq_size, slot_count, word_length, max_ix, c->own_blob, stats);
+                if (r) return fail(c, r, urmb_build_last_error());
+                if (stats[1])
+                    return fail(c, URMB_E_OVERFLOW, std::to_string(stats[1]) + " list(s) would have to be truncated (TruncateSlot)");
+                const double d = now();
+                t_build[i] = d - b;
+                urmb_index_desc desc{word_length, max_ix, (uint32_t)tabs[i].seq_size, 0, slot_count, c->own_blob, c->own_seq};
+                r = set_index(c, &desc);
+                t_pack[i] = now() - d;
+                return r;
+            }();
+        });
+    for (auto &t : th) t.join();
+    for (int i = 0; i < n; ++i)
+        if (rcs[i]) return fail(c, rcs[i], ctxs[i]->err);
+    urmb_index_host *h = new urmb_index_host;
+    const FastaTable &t = tabs[0];
+    h->word_length = word_length;
+    h->max_ix = max_ix;
+    h->seq_data_size = (uint32_t)t.seq_size;
+    h->slot_count = slot_count;
+    for (const std::string &l : t.labels) h->labels.push_back(std::string(l.c_str()));   // as urmb_index_load_host reads them
+    h->lengths = t.lengths;
+    h->offsets = t.offsets;
+    h->dropped = t.dropped;
+    h->fasta_times[0] = t1 - t0;
+    for (int i = 0; i < n; ++i) {
+        h->fasta_times[1] = std::max(h->fasta_times[1], t_parse[i]);
+        h->fasta_times[2] = std::max(h->fasta_times[2], t_build[i]);
+        h->fasta_times[3] = std::max(h->fasta_times[3], t_pack[i]);
+        h->fasta_times[4] = std::max(h->fasta_times[4], (double)k_ms[i] / 1e3);
+    }
+    *header = h;
+    return URMB_OK;
+}
+
+extern "C" int urmb_index_dropped(const urmb_index_host *h, uint32_t i, const char **label) {
+    if (!h || !label || i >= h->dropped.size()) return URMB_E_ARG;
+    *label = h->dropped[i].c_str();
+    return URMB_OK;
+}
+
+extern "C" int urmb_index_fasta_times(const urmb_index_host *h, double *t) {
+    if (!h || !t) return URMB_E_ARG;
+    memcpy(t, h->fasta_times, sizeof h->fasta_times);
     return URMB_OK;
 }
 

@@ -533,7 +533,7 @@ __global__ void build_repair_kernel(BuildArgs a) {
     }
 }
 
-static std::string g_build_err;
+static thread_local std::string g_build_err;   // per thread: urmb_index_from_fasta builds on several GPUs at once
 
 #define BCK(call)                                                                          \
     do {                                                                                   \

@@ -5,6 +5,8 @@
 //   urmap_b200 -make_ufi ref.fa -output ref.ufi [-wordlength 24] [-maxix 32] [-slots N] [-load_factor 0.6] [-veryfast] [-gpu_build]
 //   urmap_b200 -map reads.fq[.gz] -ufi ref.ufi -samout out.sam [-threads N] [-veryfast] [-gpus G] [-batch N]
 //   urmap_b200 -map2 R1.fq -reverse R2.fq -ufi ref.ufi -samout out.sam [-tabbedout out.tab] [-threads N] [-veryfast] [-minq 10]
+//   urmap_b200 -map / -map2 ... -ref ref.fa[.gz] [-wordlength 24] [-maxix 32] [-slots N] [-load_factor 0.6] (index built on the
+//              GPU(s) at start-up, the table -make_ufi writes for the same options; no UFI file)
 //   urmap_b200 -ufi_info ref.ufi
 //   urmap_b200 -ufi_validate ref.ufi          (also: -make_ufi ... -validate)
 //
@@ -94,7 +96,7 @@ static double now_s() {
 // options
 // ------------------------------------------------------------------------------------------------
 struct Opts {
-    std::string make_ufi, map, map2, reverse, ufi, samout, output, log, slots, ufi_info, ufi_validate, fastq_dump, sam_bench, tabbedout;
+    std::string make_ufi, map, map2, reverse, ufi, ref, samout, output, log, slots, ufi_info, ufi_validate, fastq_dump, sam_bench, tabbedout;
     unsigned threads = 0, wordlength = 24, maxix = 32, minq = 10, gpus = 1, batch = 262144;
     double load_factor = 0.6;
     bool veryfast = false, quiet = false, gpu_build = false, version = false, validate = false;
@@ -166,6 +168,7 @@ static Opts ParseCmdLine(int argc, char **argv) {
         else if (name == "fastq_dump") o.fastq_dump = val();
         else if (name == "sam_bench") o.sam_bench = val();
         else if (name == "ufi") o.ufi = val();
+        else if (name == "ref") o.ref = val();
         else if (name == "samout") o.samout = val();
         else if (name == "tabbedout") o.tabbedout = val();
         else if (name == "output") o.output = val();
@@ -1202,11 +1205,14 @@ static std::string MemBytesToStr(double Bytes);
 // CheckUsedOpts (cmdline.cpp:13-26, urmap_main.cpp:37): after a command that ends normally every option that was given but
 // never looked at gets "WARNING: Option -x not used", in the order of myopts.h.  Which options a command looks at was taken
 // from the reference binary itself, one extra option at a time; the output files, -log and -quiet count as used everywhere
-// (main opens them), and so do this program's own options (-gpus, -batch, -gpu_build; -threads with -ufi_validate).
+// (main opens them), and so do this program's own options (-gpus, -batch, -gpu_build, -ref; -threads with -ufi_validate).
+// With -ref the index options (-slots, -wordlength, -maxix, -load_factor) are used as -make_ufi uses them.
 static void WarnUnusedOpts(const Opts &o, const char *cmd) {
     static const char *order[] = {"slots", "ufi", "reverse", "threads", "wordlength", "minq", "maxix", "load_factor", "validate", "veryfast"};
     const std::string c = cmd;
     auto used = [&](const std::string &n) {
+        if ((c == "map" || c == "map2") && !o.ref.empty() && (n == "slots" || n == "wordlength" || n == "maxix" || n == "load_factor"))
+            return true;
         if (c == "make_ufi") return n == "slots" || n == "wordlength" || n == "maxix" || n == "load_factor" || n == "validate" || n == "veryfast";
         if (c == "map") return n == "ufi" || n == "threads" || n == "veryfast";
         if (c == "map2") return n == "ufi" || n == "reverse" || n == "threads" || n == "minq" || n == "veryfast";
@@ -1236,24 +1242,87 @@ static void FinishRun(const Opts &o, const char *cmd) {
     }
 }
 
+// The table the index options select for a FASTA file (cmd_make_ufi, ufindexio.cpp:117-179): -make_ufi and -ref both take it
+// from here, so that `-ref g.fa <opts>` maps with the table of `-make_ufi g.fa <opts>`.
+struct IndexShape {
+    uint32_t W = 24, MaxIx = 32;
+    uint64_t SlotCount = 0;
+    int64_t GenomeSize = 0;   // bytes of the file on disk (compressed, for a .gz file)
+};
+static IndexShape IndexShapeFor(const Opts &o, const std::string &fasta);
+
+// Whole FASTA file in memory for -ref: plain files are mapped, gzip files (magic 1f 8b, as gzopen tells them apart) are
+// inflated on the host into one buffer.
+struct RawFile {
+    const uint8_t *p = nullptr;
+    size_t n = 0;
+    void *map = nullptr;
+    std::vector<uint8_t> buf;
+    explicit RawFile(const std::string &path) {
+        const int fd = open(path.c_str(), O_RDONLY);
+        if (fd < 0) Die("Cannot open %s", path.c_str());
+        struct stat sb;
+        if (fstat(fd, &sb) != 0) Die("Cannot stat %s", path.c_str());
+        uint8_t magic[2] = {0, 0};
+        const bool gz = pread(fd, magic, 2, 0) == 2 && magic[0] == 0x1f && magic[1] == 0x8b;
+        if (!gz) {
+            n = (size_t)sb.st_size;
+            if (n) {
+                map = mmap(nullptr, n, PROT_READ, MAP_PRIVATE | MAP_POPULATE, fd, 0);
+                if (map == MAP_FAILED) Die("Cannot map %s", path.c_str());
+                p = (const uint8_t *)map;
+            }
+            close(fd);
+            return;
+        }
+        gzFile g = gzdopen(fd, "rb");
+        if (!g) Die("Cannot open %s", path.c_str());
+        gzbuffer(g, 1 << 20);
+        size_t cap = std::max<size_t>((size_t)sb.st_size * 4, 1 << 20);
+        for (;;) {
+            buf.resize(cap);
+            while (n < cap) {
+                const unsigned want = (unsigned)std::min<size_t>(cap - n, 1u << 30);
+                const int r = gzread(g, buf.data() + n, want);
+                if (r < 0) Die("Read error in %s", path.c_str());
+                if (r == 0) break;
+                n += (size_t)r;
+            }
+            if (n < cap) break;
+            cap *= 2;
+        }
+        gzclose(g);
+        buf.resize(n);
+        p = buf.data();
+    }
+    ~RawFile() { if (map) munmap(map, n); }
+};
+
 static int CmdMap(const Opts &o, bool paired) {
-    if (o.ufi.empty()) Die("-ufi required");
+    if (o.ufi.empty() && o.ref.empty()) Die("-ufi required (or -ref)");
+    if (!o.ufi.empty() && !o.ref.empty()) Die("-ufi and -ref are mutually exclusive");
     if (paired && o.reverse.empty()) Die("-reverse required");  // map2.cpp:42
     const double t_start = now_s();
     urmb_index_host *hix = nullptr;
-    if (urmb_index_load_host(o.ufi.c_str(), &hix) != 0) Die("%s", urmb_last_error(nullptr));
+    IndexShape X;
+    if (!o.ref.empty()) X = IndexShapeFor(o, o.ref);
+    else if (urmb_index_load_host(o.ufi.c_str(), &hix) != 0) Die("%s", urmb_last_error(nullptr));
     urmb_index_desc d;
     uint32_t ncontig = 0;
-    urmb_index_info(hix, &d, &ncontig);
     Contigs C;
-    for (uint32_t i = 0; i < ncontig; ++i) {
-        urmb_contig c;
-        urmb_index_contig(hix, i, &c);
-        C.labels.push_back(c.label);
-        C.lengths.push_back(c.length);
-        C.offsets.push_back(c.offset);
-    }
-    if (o.veryfast && d.max_ix > 3) fprintf(stderr, "\nWARNING: index not optimal for -veryfast\n\n");  // map.cpp:49
+    auto read_contigs = [&]() {   // the contig table of a UFI file or of the index built from -ref
+        urmb_index_info(hix, &d, &ncontig);
+        for (uint32_t i = 0; i < ncontig; ++i) {
+            urmb_contig c;
+            urmb_index_contig(hix, i, &c);
+            C.labels.push_back(c.label);
+            C.lengths.push_back(c.length);
+            C.offsets.push_back(c.offset);
+        }
+    };
+    if (hix) read_contigs();
+    const uint32_t word_length = hix ? d.word_length : X.W, max_ix = hix ? d.max_ix : X.MaxIx;
+    if (o.veryfast && max_ix > 3) fprintf(stderr, "\nWARNING: index not optimal for -veryfast\n\n");  // map.cpp:49
     urmb_params p{};
     p.method = (!paired && o.veryfast) ? 7 : 6;       // map.cpp:34-37; map2 always uses method 6 (map2.cpp:15)
     p.pe_method = (paired && o.veryfast) ? 5 : 4;     // map2.cpp:46-48
@@ -1270,7 +1339,7 @@ static int CmdMap(const Opts &o, bool paired) {
     std::vector<std::unique_ptr<HostBatch>> spare;
     std::thread prealloc([&]() {
         for (int g = 0; g < ngpu; ++g)   // slot buffers for reads of up to 160 bases; longer reads grow them later
-            if (urmb_reserve(ctxs[g], o.batch, 160, paired ? 1 : 0, d.word_length) != 0) Die("GPU %d: %s", g, urmb_last_error(ctxs[g]));
+            if (urmb_reserve(ctxs[g], o.batch, 160, paired ? 1 : 0, word_length) != 0) Die("GPU %d: %s", g, urmb_last_error(ctxs[g]));
         const int want = (paired ? 2 : 1) * (6 + ngpu * URMB_SLOTS);
         for (int i = 0; i < want; ++i) {
             std::unique_ptr<HostBatch> b(new HostBatch);
@@ -1279,10 +1348,30 @@ static int CmdMap(const Opts &o, bool paired) {
             spare.push_back(std::move(b));
         }
     });
-    if (urmb_index_broadcast(ctxs.data(), ngpu, hix) != 0) Die("index upload: %s", urmb_last_error(ctxs[0]));
+    if (hix) {
+        if (urmb_index_broadcast(ctxs.data(), ngpu, hix) != 0) Die("index upload: %s", urmb_last_error(ctxs[0]));
+    } else {
+        std::unique_ptr<RawFile> fa(new RawFile(o.ref));
+        const double t_read = now_s();
+        const int rc = urmb_index_from_fasta(ctxs.data(), ngpu, fa->p, fa->n, X.W, X.MaxIx, X.SlotCount, &hix);
+        if (rc == URMB_E_IO) Die("Bad FASTA file %s, %s", o.ref.c_str(), urmb_last_error(ctxs[0]));
+        if (rc == URMB_E_OVERFLOW || rc == URMB_E_UNSUPPORTED)
+            Die("GPU index build of %s: %s; build the index with -make_ufi (it builds every table on the host) and map with -ufi",
+                o.ref.c_str(), urmb_last_error(ctxs[0]));
+        if (rc != 0) Die("index from %s: %s", o.ref.c_str(), urmb_last_error(ctxs[0]));
+        fa.reset();
+        const char *lab;
+        for (uint32_t i = 0; urmb_index_dropped(hix, i, &lab) == 0; ++i)
+            fprintf(stderr, "\nWARNING: Empty sequence in FASTA file %s, label >%s\n\n", o.ref.c_str(), lab);   // as -make_ufi
+        double t[5];
+        urmb_index_fasta_times(hix, t);
+        read_contigs();
+        Progress("Index of %s built on %d GPU(s): read %.1f s, upload %.1f s, parse %.2f s (kernels %.4f s), build %.2f s, "
+                 "total %.1f s\n", o.ref.c_str(), ngpu, t_read - t_start, t[0], t[1], t[4], t[2], now_s() - t_start);
+    }
     prealloc.join();
     const double t_loaded = now_s();
-    Progress("Index %s loaded into %d GPU(s) in %.1f s\n", o.ufi.c_str(), ngpu, t_loaded - t_start);
+    if (o.ref.empty()) Progress("Index %s loaded into %d GPU(s) in %.1f s\n", o.ufi.c_str(), ngpu, t_loaded - t_start);
 
     int nthreads = o.set_threads ? (int)o.threads : std::min((int)std::thread::hardware_concurrency(), 32);
     if (nthreads < 1) nthreads = 1;
@@ -1705,23 +1794,33 @@ struct UfiBuilder {
     }
 };
 
+static IndexShape IndexShapeFor(const Opts &o, const std::string &fasta) {
+    IndexShape x;
+    x.W = o.set_wordlength ? o.wordlength : 24;
+    x.MaxIx = o.veryfast ? 3 : 32;
+    if (o.set_maxix) x.MaxIx = o.maxix;
+    FILE *f = fopen(fasta.c_str(), "rb");
+    if (!f) Die("Cannot open %s", fasta.c_str());
+    fseeko(f, 0, SEEK_END);
+    x.GenomeSize = ftello(f);
+    fclose(f);
+    if (!o.slots.empty()) x.SlotCount = strtoull(o.slots.c_str(), nullptr, 10);
+    else x.SlotCount = GetPrime((uint64_t)(int64_t)(x.GenomeSize / o.load_factor));
+    if (x.GenomeSize > (int64_t)UINT32_MAX - 100000) Die("Genome too big (%lld)", (long long)x.GenomeSize);
+    return x;
+}
+
 extern "C" int urmb_host_gpu_build(const uint8_t *seq, uint64_t n, uint64_t slots, uint32_t W, uint32_t maxix, uint8_t *blob);
 static std::string ValidateTable(const uint8_t *Blob, const uint8_t *Seq, uint64_t SlotCount, uint32_t SeqDataSize, uint32_t W,
                                  uint32_t MaxIx, int nthreads);
 
 static int CmdMakeUfi(const Opts &o) {  // cmd_make_ufi, ufindexio.cpp:117-179
     UfiBuilder B;
-    B.W = o.set_wordlength ? o.wordlength : 24;
-    B.MaxIx = o.veryfast ? 3 : 32;
-    if (o.set_maxix) B.MaxIx = o.maxix;
-    FILE *f = fopen(o.make_ufi.c_str(), "rb");
-    if (!f) Die("Cannot open %s", o.make_ufi.c_str());
-    fseeko(f, 0, SEEK_END);
-    int64_t GenomeSize = ftello(f);
-    fclose(f);
-    if (!o.slots.empty()) B.SlotCount = strtoull(o.slots.c_str(), nullptr, 10);
-    else B.SlotCount = GetPrime((uint64_t)(int64_t)(GenomeSize / o.load_factor));
-    if (GenomeSize > (int64_t)UINT32_MAX - 100000) Die("Genome too big (%lld)", (long long)GenomeSize);
+    const IndexShape X = IndexShapeFor(o, o.make_ufi);
+    const int64_t GenomeSize = X.GenomeSize;
+    B.W = X.W;
+    B.MaxIx = X.MaxIx;
+    B.SlotCount = X.SlotCount;
     B.ShiftMask = B.W >= 32 ? ~0ull : ((1ull << (2 * B.W)) - 1);
     Progress("\n  Genome size  %lld\n        Slots  %llu\n  Load factor  %.2f\n  Word length  %u\n   Max abund.  %u\n\n",
              (long long)GenomeSize, (unsigned long long)B.SlotCount, GenomeSize / (double)B.SlotCount, B.W, B.MaxIx);

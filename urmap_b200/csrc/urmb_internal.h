@@ -2,6 +2,9 @@
 #pragma once
 #include <stdint.h>
 
+#include <string>
+#include <vector>
+
 #include "../../include/urmb.h"
 
 // The kernels are compiled twice: namespace urmb with the capacities every read normally fits into, and namespace urmb_big
@@ -241,5 +244,25 @@ size_t packed_words(size_t n_bytes);
 // seqc holds coarse_words(n_bytes) words and must be zero-filled before the launch
 size_t coarse_words(size_t n_bytes);
 int launch_pack_genome(const uint8_t *seq, size_t n_bytes, uint64_t *seq2, uint32_t *seqx, uint32_t *seqc, void *stream);
+
+// implemented in urmb_fasta.cu: FASTA bytes -> SeqData (UfiBuilder::ReadFasta of urmb_host.cpp)
+struct FastaTable {
+    std::vector<std::string> labels, dropped;   // labels as the file has them (NUL bytes included): kept / dropped records
+    std::vector<uint32_t> lengths, offsets;     // kept records: length and offset in SeqData
+    std::vector<uint64_t> nstart;               // kept records: kept-byte index of the first byte
+    uint64_t seq_size = 0;                      // SeqData bytes
+};
+// The parse reads whole tiles: the device buffer holds the len raw bytes, then zero bytes up to fasta_padded_len(len).
+uint64_t fasta_padded_len(uint64_t len);
+// Lines before the first header (at position first) must be empty after '\r' removal: "" or "expected '>' in line N".
+std::string fasta_check_head(const uint8_t *fa, uint64_t first);
+// Header starts h[0..R] (h[R] = len), their line ends e[0..R) and K[0..R], the kept bytes before each header (K[R]: all of
+// them) -> record table; "" or an error message.
+std::string fasta_table(const uint8_t *fa, const uint64_t *h, const uint64_t *e, const uint64_t *K, uint64_t R, FastaTable &t);
+// Parses d_fa (len raw bytes, padded) on the current device, on stream st.  On success *d_seq is a new buffer with SeqData and
+// URMB_SEQ_PAD zero bytes and *kernel_ms the device time of the parse; h_fa: the same bytes on the host (labels, lines before
+// the first header).  Errors: URMB_E_IO (bad FASTA, no sequence), URMB_E_UNSUPPORTED (too big), URMB_E_CUDA / URMB_E_NOMEM.
+int fasta_parse_device(const uint8_t *d_fa, const uint8_t *h_fa, uint64_t len, void *st, void **d_seq, FastaTable &tab,
+                       float *kernel_ms, std::string &err);
 
 }  // namespace URMB_NS

@@ -74,7 +74,8 @@ EXPORTS = [
     "urmb_launch", "urmb_download", "urmb_timing_last", "urmb_launch_count", "urmb_mark", "urmb_mark_elapsed",
     "urmb_build_index_device", "urmb_build_last_error", "urmb_peak_gather", "urmb_peak_alu",
     "urmb_host_alloc", "urmb_host_free", "urmb_reserve", "urmb_second_hits", "urmb_overflow_count",
-    "urmb_unsupported_count", "urmb_first_look_count",
+    "urmb_unsupported_count", "urmb_first_look_count", "urmb_index_from_fasta", "urmb_index_dropped",
+    "urmb_index_fasta_times",
 ]
 
 _lib = None
@@ -123,6 +124,10 @@ def lib():
         L.urmb_host_alloc.argtypes = [C.c_size_t, C.POINTER(vp)]
         L.urmb_host_free.argtypes = [vp]
         L.urmb_host_free.restype = None
+        L.urmb_index_from_fasta.argtypes = [C.POINTER(vp), C.c_int, vp, C.c_uint64, C.c_uint32, C.c_uint32, C.c_uint64,
+                                            C.POINTER(vp)]
+        L.urmb_index_dropped.argtypes = [vp, C.c_uint32, C.POINTER(C.c_char_p)]
+        L.urmb_index_fasta_times.argtypes = [vp, C.POINTER(C.c_double)]
         for nm in EXPORTS:
             if nm not in ("urmb_last_error", "urmb_launch_count", "urmb_index_free_host", "urmb_ctx_destroy",
                           "urmb_build_last_error", "urmb_host_free"):
@@ -217,6 +222,50 @@ class Context:
         d = IndexDesc(word_length, max_ix, seq_data_size, 0, slot_count, d_blob_ptr, d_seq_ptr)
         _check(lib().urmb_index_attach(self.c, C.byref(d)), self.c)
         self._keep = list(keepalive)
+
+    def index_from_fasta(self, path: str, word_length: int = 24, max_ix: int = 32, slot_count: int | None = None,
+                         load_factor: float = 0.6):
+        """Build the index of a FASTA file (plain or gzip) on this GPU: the table `-make_ufi` writes for the same options,
+        without a file.  slot_count defaults to -make_ufi's: the first table prime >= file size / load_factor.  Returns the
+        contig list in the form of HostIndex.contigs; self.dropped lists the labels of the records without sequence."""
+        import gzip
+        from .index_build import get_prime
+        if slot_count is None:
+            slot_count = get_prime(int(os.path.getsize(path) / load_factor))
+        with open(path, "rb") as f:
+            data = f.read()
+        if data[:2] == b"\x1f\x8b":
+            data = gzip.decompress(data)
+        buf = np.frombuffer(data, dtype=np.uint8) if data else np.zeros(1, dtype=np.uint8)
+        ctxs = (C.c_void_p * 1)(self.c)
+        h = C.c_void_p()
+        _check(lib().urmb_index_from_fasta(ctxs, 1, buf.ctypes.data, len(data), word_length, max_ix, slot_count, C.byref(h)),
+               self.c)
+        try:
+            n = C.c_uint32()
+            _check(lib().urmb_index_info(h, None, C.byref(n)))
+            contigs = []
+            for i in range(n.value):
+                c = Contig()
+                _check(lib().urmb_index_contig(h, i, C.byref(c)))
+                contigs.append((c.label.decode(), c.length, c.offset))
+            self.dropped = []
+            lab = C.c_char_p()
+            while lib().urmb_index_dropped(h, len(self.dropped), C.byref(lab)) == 0:
+                self.dropped.append(lab.value.decode())
+            t = (C.c_double * 5)()
+            _check(lib().urmb_index_fasta_times(h, t))
+            self.fasta_times = dict(zip(("upload_s", "parse_s", "build_s", "pack_s", "parse_kernel_s"), list(t)))
+        finally:
+            lib().urmb_index_free_host(h)
+        self._keep = []
+        return contigs
+
+    def device_index(self) -> IndexDesc:
+        """Description of the index the context maps against (device pointers)."""
+        d = IndexDesc()
+        _check(lib().urmb_index_device_desc(self.c, C.byref(d)), self.c)
+        return d
 
     # -- State1::Search / State2::Search over a whole batch -----------------------------
     def map_se(self, seqs, offs):
